@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                      # this repo's sm_100a path, workload A (config 2)
     python bench.py --workload A101 | B                                 # R101 (config 3) | 544x544 bs=32 (config 4)
     python bench.py --impl reference --gpus N --steps K --warmup W      # the reference's CPU forward (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR             # + the last timed step's outputs as DIR/*.npy
 
 One "step" = one pass of the whole hot path (image -> backbone/FPN -> head -> decode/NMS -> mask assembly ->
 bit-packed masks) over one synthetic image per GPU (workload B: one 32-image batch per GPU).  Prints ONE JSON line (rank 0).
@@ -205,23 +206,26 @@ def oracle_step(net, img, wl):
     return res
 
 
-def cpu_reference(wl, steps, warmup, threads, budget_s=150.0):
+def cpu_reference(wl, steps, warmup, threads, budget_s=None):
+    """Times WHOLE images only (r1's row-strip extrapolation was refuted by its own numbers): `warmup` untimed images, then
+    `steps` timed ones.  With `budget_s` (the bounded CPU sample beside the GPU arm) the first image is a probe and both
+    counts shrink to what fits the time budget, at least one warm-up and one timed image.  Returns (seconds per image,
+    detections, images timed, per-image times, warm-up images)."""
     if wl.get('vis'):
         from oracle import postproc as P
         oracle_step.tracker = P.VISTracker()
-    """Times WHOLE images only (r1's row-strip extrapolation was refuted by its own numbers).  The first pass is the probe;
-    the number of timed images is min(steps, what fits the time budget), at least 1.  Returns (seconds per image,
-    detections, images timed, per-image times)."""
     from sipmask_b200 import synth
     net = build_oracle(wl, threads)
     img = synth.synthetic_image(wl['H'], wl['W'], seed=0)
-    t0 = time.perf_counter()
-    res = oracle_step(net, img, wl)                       # probe = first warm-up image
-    t_probe = time.perf_counter() - t0
-    n_warm = max(0, min(warmup - 1, int(0.2 * budget_s / max(t_probe, 1e-3))))
-    for _ in range(n_warm):
+    n_warm, n_timed = max(0, warmup), steps
+    if budget_s is not None:
+        t0 = time.perf_counter()
+        oracle_step(net, img, wl)                         # probe = first warm-up image
+        t_probe = max(time.perf_counter() - t0, 1e-3)
+        n_warm = 1 + max(0, min(warmup - 1, int(0.2 * budget_s / t_probe)))
+        n_timed = max(1, min(steps, int(0.8 * budget_s / t_probe)))
+    for _ in range(n_warm - (budget_s is not None)):
         oracle_step(net, img, wl)
-    n_timed = max(1, min(steps, int(0.8 * budget_s / max(t_probe, 1e-3))))
     ts, stages = [], []
     for _ in range(n_timed):
         t0 = time.perf_counter()
@@ -231,7 +235,7 @@ def cpu_reference(wl, steps, warmup, threads, budget_s=150.0):
     cpu_reference.stage_split = None
     if all(stages):                                        # median per stage over the timed images (not for the VIS workload)
         cpu_reference.stage_split = {k: round(statistics.median(st[k] for st in stages), 4) for k in stages[0]}
-    return statistics.median(ts), int(res['det_bboxes'].shape[0]), n_timed, ts, 1 + n_warm
+    return statistics.median(ts), int(res['det_bboxes'].shape[0]), n_timed, ts, n_warm
 
 
 def run_reference(args):
@@ -242,9 +246,9 @@ def run_reference(args):
     threads, tinfo = host_threads()
     sec, ndet, n_timed, ts, n_warm = cpu_reference(wl, args.steps, args.warmup, threads)
     val = 1.0 / sec
-    sample = ('%d whole %dx%d images timed (median; of --steps %d, bounded by a 150 s budget) after %d warm-up image(s), through the '
+    sample = ('%d whole %dx%d images timed (median) after %d warm-up image(s), through the '
               'oracle = PyTorch CPU fp32 restatement of the reference forward incl. get_bboxes on %d threads; the literal '
-              'reference cannot run on CPU (DeformConv / CropSplit are CUDA-only)' % (n_timed, wl['H'], wl['W'], args.steps, n_warm, threads))
+              'reference cannot run on CPU (DeformConv / CropSplit are CUDA-only)' % (n_timed, wl['H'], wl['W'], n_warm, threads))
     line = dict(impl='reference', metric='images/sec', value=val, unit='images/s', n_gpus=args.gpus, steps=args.steps,
                 warmup=args.warmup, ms_per_step=sec * 1e3, higher_is_better=True, scaling='weak',
                 vs_baseline=None, dtype='f32', data='synthetic',
@@ -350,10 +354,11 @@ def run_ours(args):
         runner.flush(consume)                  # the timed region ends when the last result is on the host
         finish_records()
 
-    def timed(fn, steps, sample_clocks=False, finish=None):
+    def timed(fn, steps, sample_clocks=False, finish=None, after=None):
         """K steps between barrier+synchronize, CUDA events, max over ranks.  nvidia-smi samples clocks every 100 ms;
         a short timed region would get no sample, so ROLL untimed steps of the same load run before and after it and
-        the sampler stays on throughout (clocks.window says so)."""
+        the sampler stays on throughout (clocks.window says so).  `after` runs once the timed steps are complete, before
+        the untimed steps after them overwrite their outputs."""
         sampler = ClockSampler(local) if (sample_clocks and rank == 0) else None
         roll = max(1, ROLL // ips)
         if sample_clocks:
@@ -389,6 +394,8 @@ def run_ours(args):
             finish()                                # joins the images in flight / downloads and issues the end-of-run gather
         e1.record()
         torch.cuda.synchronize()
+        if after is not None:
+            after()
         if world > 1:
             dist.barrier()
         if sample_clocks:
@@ -409,7 +416,11 @@ def run_ours(args):
         step()
     step_finish()
     torch.cuda.synchronize()
-    total_ms, clocks = timed(step, args.steps, sample_clocks=True, finish=step_finish)
+    last_step = {}
+    total_ms, clocks = timed(step, args.steps, sample_clocks=True, finish=step_finish,
+                             after=(lambda: last_step.update(step_outputs(engs))) if args.dump_outputs and rank == 0 else None)
+    if last_step:
+        write_outputs(args.dump_outputs, last_step)
     ms_per_step = total_ms / args.steps
     value = world * ips * 1000.0 / ms_per_step
     for _ in range(3):
@@ -524,6 +535,50 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 48 << 20      # --dump-outputs writes at most this much
+
+
+def step_outputs(engs):
+    """What the last forward of every engine returned (the record EnginePool.consume hands to its caller), one row per
+    image in engine order, as float32 / float64 numpy arrays: count [I]; det_bboxes [I,max,5], det_labels and idxs_keep
+    [I,max], track_feats [I,max,512] (VIS only), with the rows at and past count zeroed (no forward writes them).  The
+    bit-packed masks [I,max,H,ceil(W/32)] int32 are kept as a fixed, seeded sample of their words (all of them when they
+    fit in DUMP_BYTES): mask_bits_sample [I,K] holds the words at the flat per-image positions mask_bits_index [K]."""
+    import numpy as np
+    import torch
+    recs = [e._result() for e in engs]
+
+    def cat(k):
+        return torch.cat([r[k] for r in recs], 0)
+
+    count = cat('count').long()
+    n_img, max_num = count.shape[0], recs[0]['det_bboxes'].shape[1]
+    valid = torch.arange(max_num, device=count.device).view(1, max_num) < count.view(n_img, 1)
+
+    def rows(t):
+        keep = valid.view(n_img, max_num, *([1] * (t.dim() - 2)))
+        return torch.where(keep, t, torch.zeros((), dtype=t.dtype, device=t.device))
+
+    out = dict(count=count.float(), det_bboxes=rows(cat('det_bboxes')), det_labels=rows(cat('det_labels')).float(),
+               idxs_keep=rows(cat('idxs_keep')).double())
+    if 'track_feats' in recs[0]:
+        out['track_feats'] = rows(cat('track_feats'))
+    bits = rows(cat('mask_bits')).view(n_img, -1)
+    per_img = bits.shape[1]
+    k = (DUMP_BYTES - sum(t.numel() * t.element_size() for t in out.values())) // (8 * (n_img + 1))
+    idx = np.arange(per_img) if per_img <= k else np.sort(np.random.RandomState(0).choice(per_img, k, replace=False))
+    out['mask_bits_sample'] = bits.index_select(1, torch.from_numpy(idx).to(bits.device)).double()
+    out['mask_bits_index'] = torch.from_numpy(idx.astype(np.float64))
+    return {name: t.cpu().numpy() for name, t in out.items()}
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def mask_rooflines(line, eng, pk, pk_kind, traffic, H, IMG_W):
@@ -673,7 +728,13 @@ def main():
     ap.add_argument('--in-flight', type=int, default=int(os.environ.get('SMB_IN_FLIGHT', '0')),
                     help='forwards in flight per GPU (independent forwards on separate streams); 0 = the workload default, '
                          '1 = strictly serial')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (rank 0, see step_outputs) to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:

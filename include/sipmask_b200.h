@@ -303,9 +303,12 @@ int smb_deform_im2col_multi(int num_levels, const void* const* xs, const float* 
 int smb_maxpool3x3s2(const void* x, void* y, int N, int H, int W, int C, smb_stream_t stream);
 
 /* Bilinear upsample by an integer factor, align_corners=False (sipmask_head.py:279,285), NHWC fp16,
- * writing into a channel slice of a wider tensor (out_pitch, out_choff) so torch.cat is free. */
+ * writing into a channel slice of a wider tensor (out_pitch, out_choff) so torch.cat is free.
+ * y is [N, out_h, out_w, out_pitch]: the top-left out_h x out_w (<= H*factor x W*factor) of the upsampled map, so a
+ * level whose upsampled size exceeds the P3 map it is concatenated to is cropped instead of written past y;
+ * factor 1 (a channel copy) needs out_h == H, out_w == W. */
 int smb_upsample_bilinear(const void* x, int in_pitch, void* y, int out_pitch, int out_choff,
-                          int N, int H, int W, int C, int factor, int relu, smb_stream_t stream);
+                          int N, int H, int W, int C, int factor, int out_h, int out_w, int relu, smb_stream_t stream);
 
 /* Image preparation: NCHW fp32 -> zero-padded NHWC8 fp16 [N, H+6, W+8, 8] for the 7x7/2 stem. */
 int smb_image_to_nhwc8(const float* img, void* out, int N, int H, int W, smb_stream_t stream);

@@ -296,7 +296,8 @@ def upsample_bilinear(x, factor, out=None, out_choff=0, relu=False):
     if out is None:
         out = torch.empty((N, H * factor, W * factor, C), dtype=torch.float16, device=x.device)
     L.check(L.lib().smb_upsample_bilinear(L.ptr(x), x.stride(2), L.ptr(out), out.stride(2), int(out_choff), N, H, W, C,
-                                          int(factor), int(relu), L.stream_ptr()), 'smb_upsample_bilinear')
+                                          int(factor), out.shape[1], out.shape[2], int(relu), L.stream_ptr()),
+            'smb_upsample_bilinear')
     return out
 
 

@@ -214,11 +214,11 @@ __global__ void maxpool3x3s2_kernel(const __half* __restrict__ x, __half* __rest
 // ------------------------------------------------------------------------------------ bilinear upsample
 // PyTorch upsample_bilinear2d, align_corners=False, scale_factor = factor (integer):
 //   src = max((dst + 0.5) / factor - 0.5, 0); i0 = (int)src; i1 = i0 + (i0 < in-1); l1 = src - i0
+// y is [N, Ho, Wo, out_pitch] with Ho <= H * factor, Wo <= W * factor: the top-left Ho x Wo of the upsampled map.
 __global__ void upsample_bilinear_kernel(const __half* __restrict__ x, int in_pitch, __half* __restrict__ y, int out_pitch,
-                                         int out_choff, int N, int H, int W, int C, int factor, int relu) {
+                                         int out_choff, int N, int H, int W, int C, int factor, int Ho, int Wo, int relu) {
   pdl_wait();
   const int vecs = C >> 3;
-  const int Ho = H * factor, Wo = W * factor;
   const float rs = 1.0f / (float)factor;
   const long long total = (long long)N * Ho * Wo * vecs;
   for (unsigned t = blockIdx.x * blockDim.x + threadIdx.x; t < (unsigned)total; t += blockDim.x * gridDim.x) {   // 32-bit index math: 64-bit div/mod costs ~100 instructions each
@@ -560,9 +560,10 @@ extern "C" int smb_maxpool3x3s2(const void* x, void* y, int N, int H, int W, int
 }
 
 extern "C" int smb_upsample_bilinear(const void* x, int in_pitch, void* y, int out_pitch, int out_choff, int N, int H, int W,
-                                     int C, int factor, int relu, smb_stream_t stream) {
-  SMB_CHECK_ARG(x && y && C % 8 == 0 && in_pitch % 8 == 0 && out_pitch % 8 == 0 && out_choff % 8 == 0 && factor >= 1,
-                "smb_upsample_bilinear: bad argument");
+                                     int C, int factor, int out_h, int out_w, int relu, smb_stream_t stream) {
+  SMB_CHECK_ARG(x && y && C % 8 == 0 && in_pitch % 8 == 0 && out_pitch % 8 == 0 && out_choff % 8 == 0 && factor >= 1 &&
+                out_h >= 1 && out_w >= 1 && out_h <= H * factor && out_w <= W * factor &&
+                (factor > 1 || (out_h == H && out_w == W)), "smb_upsample_bilinear: bad argument");
   if (factor == 1) {
     const long long npix = (long long)N * H * W;
     SMB_CUDA_OK(launch_pdl(copy_channels_kernel, dim3(grid_for(npix * (C / 8), 256)), dim3(256), 0, (cudaStream_t)stream,
@@ -570,9 +571,9 @@ extern "C" int smb_upsample_bilinear(const void* x, int in_pitch, void* y, int o
     SMB_LAUNCH_OK("copy_channels_kernel");
     return SMB_OK;
   }
-  const long long total = (long long)N * H * factor * W * factor * (C / 8);
+  const long long total = (long long)N * out_h * out_w * (C / 8);
   SMB_CUDA_OK(launch_pdl(upsample_bilinear_kernel, dim3(grid_for(total, 256)), dim3(256), 0, (cudaStream_t)stream, (const __half*)x,
-                         in_pitch, (__half*)y, out_pitch, out_choff, N, H, W, C, factor, relu));
+                         in_pitch, (__half*)y, out_pitch, out_choff, N, H, W, C, factor, out_h, out_w, relu));
   SMB_LAUNCH_OK("upsample_bilinear_kernel");
   return SMB_OK;
 }

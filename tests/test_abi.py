@@ -35,6 +35,17 @@ def test_ops_fail_loudly_without_cuda():
         ops.mask_assemble(torch.zeros(32, 4, 4), torch.zeros(1, 128), torch.zeros(1, 4), 0.5)
 
 
+def test_upsample_rejects_an_output_the_input_cannot_fill():
+    """smb_upsample_bilinear writes out_h x out_w <= (H*factor) x (W*factor); a larger output (or a factor-1 copy into
+    another size) is refused before any memory is touched."""
+    from sipmask_b200 import _lib
+    lib = _lib.lib()
+    p = ctypes.c_void_p(256)                       # never dereferenced: the arguments are rejected first
+    assert lib.smb_upsample_bilinear(p, 8, p, 8, 0, 1, 7, 10, 8, 2, 15, 20, 0, None) != 0
+    assert lib.smb_upsample_bilinear(p, 8, p, 8, 0, 1, 7, 10, 8, 2, 14, 21, 0, None) != 0
+    assert lib.smb_upsample_bilinear(p, 8, p, 8, 0, 1, 7, 10, 8, 1, 6, 10, 0, None) != 0
+
+
 def test_sass_contains_blackwell_instructions():
     """The conv kernel must be real tcgen05/TMA code (B200_PROFILING.md 'What proves a Blackwell-native kernel')."""
     import shutil

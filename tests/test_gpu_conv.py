@@ -212,6 +212,15 @@ def test_upsample_bilinear_matches_torch():
         torch.cuda.synchronize()
         _check(out[..., 256:512], ref.permute(0, 2, 3, 1).double(), tol=2e-3)
         assert out[..., :256].abs().max() == 0 and out[..., 512:].abs().max() == 0
+        # an output smaller than the upsampled map (a P3 map that is not exactly 2x / 4x the level): the top-left crop,
+        # and nothing written past the output
+        ho, wo = 13 * f - f + 1, 21 * f - 3
+        buf = torch.zeros(ho * wo * 768 + 4096, dtype=torch.float16, device='cuda')
+        out = buf[:ho * wo * 768].view(1, ho, wo, 768)
+        conv.upsample_bilinear(x, f, out=out, out_choff=256)
+        torch.cuda.synchronize()
+        _check(out[..., 256:512], ref[:, :, :ho, :wo].permute(0, 2, 3, 1).double(), tol=2e-3)
+        assert buf[ho * wo * 768:].abs().max() == 0
     out = torch.zeros((1, 13, 21, 768), dtype=torch.float16, device='cuda')
     conv.upsample_bilinear(x, 1, out=out, out_choff=0)
     assert torch.equal(out[..., :256], x)

@@ -199,10 +199,10 @@ def test_registry_hooks_replace_reference_entries():
     tests/golden/_ref_import.py, build container only): `type='SipMaskHead'` then builds the drop-in class, the reference
     detector's bbox_head is ours, and mmdet.ops.{CropSplit, DeformConv, nms} point at the sm_100a operators."""
     import sys
-    if not os.path.isdir('/root/reference/SipMask-mmdetection'):
-        pytest.skip('reference tree not present (GPU box): the registry is exercised in the build container')
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
     import _ref_import
+    if not os.path.isdir(_ref_import.REF_MM):
+        pytest.skip('needs the unmodified reference mmdet package (%s), which is not present here' % _ref_import.REF_MM)
     _ref_import.install()
     from mmdet.models import build_detector
     from mmdet.models.registry import HEADS

@@ -46,24 +46,23 @@ def test_nms_bm_known_answers(golden_dir):
     assert sorted(keep.tolist()) == sorted(g['bm53_gt_indices'].tolist())
 
 
-def test_nms_matches_reference_cpp():
-    """oracle.ops.nms(cmp_ge=True) == the reference's own nms_cpu.cpp (compiled into oracle/_ref)."""
-    import sys
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref')
-    sys.path.insert(0, ref_dir)
-    try:
-        import sipmask_ref_nms_cpu as ref
-    except Exception:
-        pytest.skip('oracle/_ref not built (run oracle/build.py where /root/reference exists)')
+def nms_cpp_cases():
+    """(key, dets [n,5] float32, iou threshold) of the comparison with the reference's nms_cpu.cpp."""
     rng = np.random.RandomState(0)
     for n in (1, 7, 64, 65, 300):
         xy = rng.rand(n, 2) * 200
         wh = rng.rand(n, 2) * 80 + 1
         dets = np.concatenate([xy, xy + wh, rng.rand(n, 1)], 1).astype(np.float32)
         for thr in (0.3, 0.5, 0.7):
-            a = ref.nms(torch.from_numpy(dets), thr).numpy()
-            b = O.nms(dets, thr, cmp_ge=True)
-            assert a.tolist() == b.tolist()
+            yield 'keep_%d_%g' % (n, thr), dets, thr
+
+
+def test_nms_matches_reference_cpp(golden_dir):
+    """oracle.ops.nms(cmp_ge=True) == what the reference's own nms_cpu.cpp kept on the same boxes (ref_nms_cpu.npz,
+    generator: tests/golden/gen_golden_ref_native.py)."""
+    g = _load(golden_dir, 'ref_nms_cpu.npz')
+    for key, dets, thr in nms_cpp_cases():
+        assert O.nms(dets, thr, cmp_ge=True).tolist() == g[key].tolist(), key
 
 
 def test_c_oracle_matches_numpy():
