@@ -264,6 +264,14 @@ int smb_conv_plan_set_max_ctas(smb_conv_plan_t* plan, int max_ctas);
  * `min_tiles` output tiles (default 48; <= 0 restores the default).  Small values favour fat tiles (fewer bytes through
  * L2 -> SM per FLOP), large values favour occupancy of a single stream.  Returns the previous value. */
 int smb_conv_set_min_tiles(int min_tiles);
+/* Read-only view of what the planner chose for a plan (tests pin the branch a shape is meant to reach).  Writes the
+ * first min(n, 11) of, in this order:
+ *   n_tile, n_tiles_n, tiles_m, pair (cta_group::2), cluster (CTAs per cluster), grid (CTAs launched, after
+ *   smb_conv_plan_set_max_ctas), out_tma (TMA-store epilogue), res_tma (TMA-staged residual), stage_slots,
+ *   epi_split (split epilogue chosen at plan time; smb_conv_run falls back to the lockstep epilogue when alpha != 1,
+ *   there is no bias or the bias is not 16-byte aligned), small (conv1x1_small_kernel).
+ * Returns the number of fields the library knows (11), or a negative SMB_E* code. */
+int smb_conv_plan_info(const smb_conv_plan_t* plan, int* out, int n);
 /* out = relu?( (acc + bias) * alpha + residual ); alpha carries the per-level `Scale` of fcos_reg
  * (sipmask_head.py:261, ops/scale.py:12-15). */
 int smb_conv_run(const smb_conv_plan_t* plan, const float* bias, const void* residual, void* gn_stats,

@@ -43,7 +43,7 @@ SYMBOLS = [
     'smb_crop_split_forward', 'smb_crop_split_backward', 'smb_crop_split_gt', 'smb_mask_rle_counts', 'smb_rle_to_string', 'smb_conv3x3s2_relu_f32', 'smb_mask_rescore', 'smb_nms', 'smb_decode_workspace_bytes', 'smb_decode_topk',
     'smb_multiclass_nms_workspace_bytes', 'smb_multiclass_nms', 'smb_fast_nms_workspace_bytes', 'smb_fast_nms',
     'smb_gather_rows_f32', 'smb_gather_det_inputs', 'smb_gather_track_feats', 'smb_track_step', 'smb_conv_plan_create', 'smb_conv_plan_create_multi', 'smb_conv_plan_destroy', 'smb_conv_plan_set_max_ctas', 'smb_conv_set_min_tiles',
-    'smb_conv_run',
+    'smb_conv_plan_info', 'smb_conv_run',
     'smb_groupnorm_relu_apply', 'smb_groupnorm_stats', 'smb_deform_im2col', 'smb_offset_conv1x1', 'smb_groupnorm_relu_apply_multi', 'smb_offset_conv1x1_multi', 'smb_deform_im2col_multi', 'smb_maxpool3x3s2',
     'smb_upsample_bilinear', 'smb_image_to_nhwc8', 'smb_preprocess_u8', 'smb_stem_plan_create', 'smb_stem_plan_create_s2d', 'smb_image_to_s2d16', 'smb_preprocess_u8_s2d',
 ]

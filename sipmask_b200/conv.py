@@ -68,6 +68,11 @@ def pack_stem_weight_s2d(w, bn, eps=1e-5, device=None):
     return wk, bias
 
 
+# the fields of smb_conv_plan_info, in the order the library writes them
+PLAN_INFO_FIELDS = ('n_tile', 'n_tiles_n', 'tiles_m', 'pair', 'cluster', 'grid', 'out_tma', 'res_tma', 'stage_slots',
+                    'epi_split', 'small')
+
+
 def set_min_tiles(n):
     """Planner knob for plans created afterwards (smb_conv_set_min_tiles); returns the previous value."""
     return int(L.lib().smb_conv_set_min_tiles(int(n)))
@@ -115,6 +120,14 @@ class ConvPlan(object):
     def set_max_ctas(self, n):
         L.check(L.lib().smb_conv_plan_set_max_ctas(self.handle, int(n)), 'smb_conv_plan_set_max_ctas')
         return self
+
+    def info(self):
+        """What the planner chose for this plan (smb_conv_plan_info): tile shape, pair / cluster mode, grid, epilogue."""
+        vals = (ctypes.c_int * len(PLAN_INFO_FIELDS))()
+        rc = L.lib().smb_conv_plan_info(self.handle, vals, len(PLAN_INFO_FIELDS))
+        if rc < 0:
+            L.check(rc, 'smb_conv_plan_info')
+        return dict(zip(PLAN_INFO_FIELDS, (int(v) for v in vals)))
 
     def run(self, stream=None):
         if self.dev.index != torch.cuda.current_device():        # launch on the plan's device and ITS current stream

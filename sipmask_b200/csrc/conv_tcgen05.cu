@@ -973,8 +973,10 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
               gv[0] += __shfl_xor_sync(0xffffffffu, gv[0], 8);
               gv[0] += __shfl_xor_sync(0xffffffffu, gv[0], 16);
               if (lane < 8 && tc.active) {
+                // lane partial g covers 8 channels; with 16-channel groups two adjacent partials add into one slot
                 const int g = lane >> 1, kind = lane & 1;
-                const int grp = ((n0 + cc) >> 3) + g;
+                int grp = ((n0 + cc) >> 3) + g;
+                if (p.gn_group == 16) grp >>= 1;
                 const int ngroups = p.Cout / p.gn_group;
                 unsigned long long* st = reinterpret_cast<unsigned long long*>(L.gn_stats) + ((size_t)tc.img * ngroups + grp) * 2 + kind;
                 atomicAdd(st, (unsigned long long)__float2ll_rn(gv[0] * (kind ? kGnSqScale : kGnSumScale)));
@@ -1460,7 +1462,10 @@ static int finish_plan(smb_conv_plan* pl, int Cout, int Ktotal, const void* weig
     const char* envs = getenv("SMB_CONV_STAGE_SETS");
     const int want2 = envs ? atoi(envs) == 2 : 1;
     const int st2 = (int)((194 * 1024 - 2 * (long)stage_out) / (long)stage);
-    if (p.out_tma && want2 && 2 * stage_out <= 128 * 1024 && st2 >= (kblocks < 3 ? kblocks : 3)) {
+    // operand stages that must remain: min(kblocks, 3), and never fewer than the two the pipeline needs (a one-k-block
+    // tile of 256 channels without pair mode would otherwise be left with a single stage and no plan)
+    const int min_st = kblocks < 2 ? 2 : (kblocks < 3 ? kblocks : 3);
+    if (p.out_tma && want2 && 2 * stage_out <= 128 * 1024 && st2 >= min_st) {
       p.stage_slots *= 2;
       stage_out *= 2;
     }
@@ -1748,6 +1753,16 @@ extern "C" int smb_conv_plan_set_max_ctas(smb_conv_plan_t* plan, int max_ctas) {
   if (g < c) g = c;
   if (g < plan->grid) plan->grid = g;
   return SMB_OK;
+}
+
+extern "C" int smb_conv_plan_info(const smb_conv_plan_t* plan, int* out, int n) {
+  SMB_CHECK_ARG(plan && out && n >= 0, "smb_conv_plan_info: bad argument");
+  const ConvParams& p = plan->p;
+  const int v[] = {p.n_tile, p.n_tiles_n, p.tiles_m, p.pair, p.cluster, plan->grid, p.out_tma, p.res_tma, p.stage_slots,
+                   p.epi_split, plan->small};
+  const int nv = (int)(sizeof(v) / sizeof(v[0]));
+  for (int i = 0; i < n && i < nv; ++i) out[i] = v[i];
+  return nv;
 }
 
 extern "C" int smb_conv_run(const smb_conv_plan_t* plan, const float* bias, const void* residual, void* gn_stats,

@@ -46,6 +46,13 @@ def test_upsample_rejects_an_output_the_input_cannot_fill():
     assert lib.smb_upsample_bilinear(p, 8, p, 8, 0, 1, 7, 10, 8, 1, 6, 10, 0, None) != 0
 
 
+def test_conv_plan_info_rejects_a_null_plan():
+    from sipmask_b200 import _lib, conv
+    vals = (ctypes.c_int * len(conv.PLAN_INFO_FIELDS))()
+    assert _lib.lib().smb_conv_plan_info(None, vals, len(vals)) < 0
+    assert len(conv.PLAN_INFO_FIELDS) == 11
+
+
 def test_sass_contains_blackwell_instructions():
     """The conv kernel must be real tcgen05/TMA code (B200_PROFILING.md 'What proves a Blackwell-native kernel')."""
     import shutil
